@@ -22,6 +22,9 @@ only exchange step).
   cpu_baseline : the CPU oracle port (oracle/rife46.py == the reference's PyTorch-CPU path, SURVEY.md F2) on the
                  host cores, on a bounded sample of the same clip (rank 0, N = 1 only)
 --impl reference times that CPU port alone (all host threads), same metric / config.
+--dump-outputs DIR writes the interpolated frames of the last timed step (every rank's, in rank order) to
+DIR/interpolated_frames.npy: float32 [frames, pixels, 3] at the same seeded sample of pixel positions in every frame, so
+that two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -45,6 +48,16 @@ CPU_ARCH = "4.6"
 # internal pass of 8 pairs per chunk (r02: 16 chunks of 4 pairs made every pass half as wide - the latency-bound blocks 0 / 1
 # cost the same per pass - and the step 4.7 ms slower than N = 1, whatever the transport)
 GATHER_CHUNKS = int(os.environ.get("VFI_GATHER_CHUNKS", "8"))
+DUMP_BYTES = 60_000_000              # --dump-outputs: size bound of the written sample (a 64-frame clip is 1.6 GB)
+DUMP_SEED = 0
+
+
+def frame_sample(frames, npix):
+    """[n, H, W, 3] -> float32 CPU [n, npix, 3]: the same seeded pixel positions (raster order) of every frame."""
+    import torch
+    n, h, w, c = frames.shape
+    pos = torch.randperm(h * w, generator=torch.Generator().manual_seed(DUMP_SEED))[:npix].sort().values
+    return frames.reshape(n, h * w, c).index_select(1, pos.to(frames.device)).float().cpu()
 
 
 def _peaks():
@@ -201,7 +214,13 @@ def main():
                          "[4] through tools/bench_film.py / tools/bench_sepconv.py (same JSON-line contract, own metric name)")
     ap.add_argument("--arch", default="4.6", choices=["4.6", "4.7", "4.17", "4.26"],
                     help="RIFE arch (default 4.6 = the BASELINE.json metric; the others are side measurements)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a seeded sample of the last timed step's interpolated frames to DIR/interpolated_frames.npy")
     a, extra = ap.parse_known_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.workload != "rife" or a.impl != "b200"):
+        ap.error("--dump-outputs is implemented for the default workload (--workload rife --impl b200)")
     if a.workload != "rife":  # the other model families keep their own harness; same launch convention (torchrun for N > 1)
         import runpy
         tool = {"film": "bench_film.py", "sepconv": "bench_sepconv.py", "gmfss": "bench_gmfss.py"}[a.workload]
@@ -333,6 +352,13 @@ def main():
     launches = eng.launch_count() - l0
     ms_dev = e0.elapsed_time(e1)
     clocks = sampler.stop(t_begin, t_end) if rank == 0 else None
+    if a.dump_outputs and rank == 0:   # what a caller of the timed path receives: every rank's frames, in rank order
+        import numpy as np
+        shards = [dev_out] if dist is None else list(pusher.buffer if pusher is not None else gather_list)
+        npix = min(H * W, DUMP_BYTES // (len(shards) * npairs * 3 * 4))
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        np.save(os.path.join(a.dump_outputs, "interpolated_frames.npy"),
+                torch.cat([frame_sample(s, npix) for s in shards]).numpy())
     gather_ok = None
     if dist is not None:  # what landed on rank 0 is what every rank computed (sums of each rank's first and last frame)
         mine = torch.stack([dev_out[0].double().sum(), dev_out[-1].double().sum()])

@@ -14,7 +14,8 @@ closes that gap without copying any reference source into the repo:
   3. the kernel runs on CPU tensors through ctypes exactly as ``cuda_launch`` would run it on the device
      (``args = [n, data pointers...]``, one emulated thread walking the whole grid-stride range).
 
-``tests/test_ops_ref_pinned.py`` holds ``oracle/ops_ref.py`` to these outputs, which makes the chain
+``tools/make_golden_ops.py`` stores these outputs in ``tests/golden/ops_ref_kernels.npz`` and
+``tests/test_ops_ref_pinned.py`` holds ``oracle/ops_ref.py`` to them, which makes the chain
 reference kernel source -> oracle -> sm_100a kernels (GPU tests) complete for softsplat_out, costvol_out and sepconv_out.
 ``kernel_Correlation_rearrange`` / ``_updateOutput`` (blocks of cooperating threads, shared memory, ``__syncthreads``) run
 through a second shim, ``tests/host_emu/block_emu.h``: every thread of a block is a fiber and ``__syncthreads()`` yields to

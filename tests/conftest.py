@@ -38,3 +38,17 @@ def load_pkg():
 @pytest.fixture(scope="session")
 def pkg():
     return load_pkg()
+
+
+GOLDEN_CPU_THREADS = 8
+
+
+@pytest.fixture
+def golden_cpu_threads():
+    """The reference outputs in tests/golden were made on the CPU with 8 intra-op threads.  ATen splits some fp32
+    reductions by thread count, so the oracle meets them at rounding level only when it runs with the same count."""
+    import torch
+    before = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_CPU_THREADS)
+    yield
+    torch.set_num_threads(before)

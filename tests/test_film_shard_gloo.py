@@ -33,6 +33,9 @@ CASES = [dict(n=6, multiplier=4, states=None), dict(n=7, multiplier=[2, 5, 3], s
 
 
 def _worker(rank, world, port, q):
+    # host logic only: the stand-in engines run on the CPU, so the nodes' GPU paths (Sepconv's pipelined multiplier-2
+    # path) must not engage when the machine has a GPU
+    os.environ["CUDA_VISIBLE_DEVICES"] = ""
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     sys.path.insert(0, root)

@@ -1,88 +1,85 @@
 """Pin oracle/ops_ref.py (the CPU restatements the sm_100a op kernels are checked against on the GPU) to the REFERENCE'S OWN
 kernels: the cupy kernel strings of vfi_models/ops/cupy_ops, specialised by the reference's own pre-processor and executed
-on the CPU through tests/host_emu (oracle/ref_ops.py).  Runs in the build container only (/root/reference)."""
+on the CPU through tests/host_emu (oracle/ref_ops.py).  Their inputs and outputs are stored in
+tests/golden/ops_ref_kernels.npz (tools/make_golden_ops.py), so these tests need no copy of the reference."""
+import os
+import sys
+
+import numpy as np
 import pytest
 import torch
 
-from oracle import ops_ref, ref_ops
+from oracle import ops_ref
 
-pytestmark = pytest.mark.skipif(not ref_ops.available(), reason="/root/reference (or the CUDA headers) not present")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "tools"))
+from make_golden_ops import ADACOF, CORRELATION, COSTVOL, NPZ, SEPCONV, SOFTSPLAT, case  # noqa: E402
+
+_GOLD = np.load(NPZ)
 
 
-@pytest.mark.parametrize("shape,mag", [((1, 3, 9, 13), 1.5), ((2, 5, 8, 8), 6.0)])
+def golden(name):
+    prefix = name + ":"
+    d = {k[len(prefix):]: torch.from_numpy(_GOLD[k]) for k in _GOLD.files if k.startswith(prefix)}
+    assert d, name
+    return d
+
+
+@pytest.mark.parametrize("shape,mag", SOFTSPLAT)
 def test_softsplat_sum_matches_reference_kernel(shape, mag):
-    g = torch.Generator().manual_seed(shape[1])
-    x = torch.randn(*shape, generator=g)
-    flow = (torch.rand(shape[0], 2, shape[2], shape[3], generator=g) - 0.5) * 2 * mag   # some targets fall outside
-    ref = ref_ops.softsplat_out(x, flow)
-    got = ops_ref.softsplat_sum(x, flow)
-    assert (got - ref).abs().max().item() <= 1e-5
+    g = golden(case("softsplat_sum", shape, mag))
+    got = ops_ref.softsplat_sum(g["x"], g["flow"])
+    assert (got - g["out"]).abs().max().item() <= 1e-5
 
 
 def test_softsplat_modes_on_top_of_the_reference_kernel():
     """softsplat() (cupy_ops/softsplat.py:382-435) = host arithmetic around softsplat_out; with the kernel being the
     reference's, 'avg' and 'soft' of the oracle must agree with that arithmetic done here."""
-    g = torch.Generator().manual_seed(1)
-    x = torch.randn(1, 4, 7, 9, generator=g)
-    flow = (torch.rand(1, 2, 7, 9, generator=g) - 0.5) * 5
-    metric = torch.randn(1, 1, 7, 9, generator=g) * 0.3
-    avg_in = torch.cat([x, x.new_ones(1, 1, 7, 9)], 1)
-    o = ref_ops.softsplat_out(avg_in, flow)
+    g = golden("softsplat_modes")
+    x, flow, metric = g["x"], g["flow"], g["metric"]
+    o = g["avg"]
     norm = o[:, -1:].clone()
     norm[norm == 0.0] = 1.0
     assert (ops_ref.softsplat(x, flow, None, "avg") - o[:, :-1] / norm).abs().max().item() <= 2e-4  # small normalisers amplify fp32 rounding
-    soft_in = torch.cat([x * metric.exp(), metric.exp()], 1)
-    o = ref_ops.softsplat_out(soft_in, flow)
+    o = g["soft"]
     norm = o[:, -1:].clone()
     norm[norm == 0.0] = 1.0
     assert (ops_ref.softsplat(x, flow, metric, "soft") - o[:, :-1] / norm).abs().max().item() <= 2e-4  # small normalisers amplify fp32 rounding
 
 
-@pytest.mark.parametrize("shape", [(1, 8, 6, 7), (2, 3, 10, 5)])
+@pytest.mark.parametrize("shape", COSTVOL)
 def test_costvol_matches_reference_kernel(shape):
-    g = torch.Generator().manual_seed(shape[2])
-    one, two = torch.randn(*shape, generator=g), torch.randn(*shape, generator=g)
-    assert (ops_ref.costvol_l1(one, two) - ref_ops.costvol_out(one, two)).abs().max().item() <= 1e-5
+    g = golden(case("costvol", shape))
+    assert (ops_ref.costvol_l1(g["one"], g["two"]) - g["out"]).abs().max().item() <= 1e-5
 
 
-@pytest.mark.parametrize("k,hw", [(5, (6, 7)), (51, (4, 3))])
+@pytest.mark.parametrize("k,hw", SEPCONV)
 def test_sepconv_matches_reference_kernel(k, hw):
-    g = torch.Generator().manual_seed(k)
-    x = torch.randn(1, 4, hw[0] + k - 1, hw[1] + k - 1, generator=g)
-    ver, hor = torch.randn(1, k, *hw, generator=g), torch.randn(1, k, *hw, generator=g)
-    ref = ref_ops.sepconv_out(x, ver, hor)
-    got = ops_ref.sepconv(x, ver, hor)
+    g = golden(case("sepconv", k, hw))
+    ref = g["out"]
+    got = ops_ref.sepconv(g["x"], g["ver"], g["hor"])
     assert (got - ref).abs().max().item() <= 1e-4 * max(1.0, float(ref.abs().max()))
 
 
-@pytest.mark.parametrize("shape", [(1, 40, 5, 6), (2, 7, 4, 9)])
+@pytest.mark.parametrize("shape", CORRELATION)
 def test_correlation_dot_matches_reference_kernels(shape):
     """kernel_Correlation_rearrange + kernel_Correlation_updateOutput with blocks of 16 / 32 cooperating threads (fibers)."""
-    g = torch.Generator().manual_seed(shape[1])
-    a, b = torch.randn(*shape, generator=g), torch.randn(*shape, generator=g)
-    ref = ref_ops.correlation(a, b)
-    assert (ops_ref.correlation_dot(a, b) - ref).abs().max().item() <= 1e-5
+    g = golden(case("correlation", shape))
+    assert (ops_ref.correlation_dot(g["a"], g["b"]) - g["out"]).abs().max().item() <= 1e-5
 
 
-@pytest.mark.parametrize("f,dil", [(3, 1), (5, 2)])
+@pytest.mark.parametrize("f,dil", ADACOF)
 def test_adacof_matches_reference_kernel(f, dil):
-    g = torch.Generator().manual_seed(f)
-    n, c, ho, wo = 2, 3, 6, 7
-    x = torch.randn(n, c, ho + (f - 1) * dil, wo + (f - 1) * dil, generator=g)
-    w = torch.randn(n, f * f, ho, wo, generator=g)
-    oi = torch.randn(n, f * f, ho, wo, generator=g) * 2.5      # negative offsets: (int) truncation != floor
-    oj = torch.randn(n, f * f, ho, wo, generator=g) * 2.5
-    ref = ref_ops.adacof(x, w, oi, oj, dil)
-    assert (ops_ref.adacof(x, w, oi, oj, dil) - ref).abs().max().item() <= 2e-5 * max(1.0, float(ref.abs().max()))
+    g = golden(case("adacof", f, dil))
+    ref = g["out"]
+    assert (ops_ref.adacof(g["x"], g["w"], g["oi"], g["oj"], dil) - ref).abs().max().item() <= 2e-5 * max(1.0, float(ref.abs().max()))
 
 
 def test_edt_matches_reference_kernel_and_scipy():
-    g = torch.Generator().manual_seed(2)
-    img = (torch.rand(2, 9, 12, generator=g) > 0.85).float()
-    img[1] = 0                                                   # empty image: defaults to the diameter
+    g = golden("edt")
+    img, data = g["img"], g["data"]
     diam2 = 9 ** 2 + 12 ** 2
-    data = (1 - img) * diam2
-    assert torch.equal(ops_ref.edt_pass(data, diam2), ref_ops.edt_pass(data, diam2))
+    assert torch.equal(ops_ref.edt_pass(data, diam2), g["out"])
     from scipy import ndimage
     want = ndimage.distance_transform_edt(1 - img[0].numpy())
     assert abs(ops_ref.batch_edt(img)[0].numpy() - want).max() <= 1e-4

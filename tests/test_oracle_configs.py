@@ -6,6 +6,7 @@ import os
 import sys
 
 import numpy as np
+import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -14,6 +15,7 @@ from make_golden_configs import CFG1, CFG2, CROP, box8, crop_origins  # noqa: E4
 from oracle import rife46 as O  # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
+pytestmark = pytest.mark.usefixtures("golden_cpu_threads")
 QSTEP = 1.0 / 65535.0
 
 

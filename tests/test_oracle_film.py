@@ -13,6 +13,7 @@ from make_golden_film import film_cases, film_inputs  # noqa: E402
 from oracle import film as OF  # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
+pytestmark = pytest.mark.usefixtures("golden_cpu_threads")
 
 
 @pytest.mark.parametrize("name", sorted(film_cases().keys()))

@@ -13,6 +13,7 @@ from make_golden import cases, make_inputs  # noqa: E402
 from oracle import rife46 as O  # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
+pytestmark = pytest.mark.usefixtures("golden_cpu_threads")
 
 
 @pytest.mark.parametrize("name", sorted(cases().keys()))
