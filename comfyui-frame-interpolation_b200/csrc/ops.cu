@@ -16,6 +16,18 @@
 namespace vfi {
 namespace {
 
+// Top-left corner (x0, y0) of the four targets of a splat source moved to (fx, fy); false when none of them is in the
+// image.  The test is made on the floored floats, so the int conversion only sees values in [-1, W) x [-1, H): a flow of
+// 2^31 or more converts to INT_MAX on the GPU (saturation), and x0 + 1 would then overflow, which the compiler is free to
+// assume never happens (it tests x0 + 1 >= 0 as x0 > -2 next to a wrapped x0 + 1 < W, accepting x1 = INT_MIN).
+__device__ __forceinline__ bool splat_corner(float fx, float fy, int W, int H, int& x0, int& y0) {
+  const float lx = floorf(fx), ly = floorf(fy);
+  if (!(lx >= -1.f && lx < (float)W && ly >= -1.f && ly < (float)H)) return false;
+  x0 = (int)lx;
+  y0 = (int)ly;
+  return true;
+}
+
 __global__ void softsplat_sum_kernel(const float* __restrict__ in, const float* __restrict__ flow,
                                      float* __restrict__ out, int N, int C, int H, int W) {
   const size_t hw = (size_t)H * W;
@@ -28,7 +40,8 @@ __global__ void softsplat_sum_kernel(const float* __restrict__ in, const float* 
     const float fx = (float)x + __ldg(flow + ((size_t)n * 2 + 0) * hw + pix);
     const float fy = (float)y + __ldg(flow + ((size_t)n * 2 + 1) * hw + pix);
     if (!isfinite(fx) || !isfinite(fy)) continue;  // softsplat.py:158-159
-    const int x0 = (int)floorf(fx), y0 = (int)floorf(fy);
+    int x0, y0;
+    if (!splat_corner(fx, fy, W, H, x0, y0)) continue;
     const int x1 = x0 + 1, y1 = y0 + 1;
     const float wnw = ((float)x1 - fx) * ((float)y1 - fy);
     const float wne = (fx - (float)x0) * ((float)y1 - fy);
@@ -67,7 +80,8 @@ __global__ void softsplat_weighted_kernel(const float* __restrict__ in, const fl
     const float fy = (float)y + __ldg(flow + ((size_t)n * 2 + 1) * hw + pix);
     if (!isfinite(fx) || !isfinite(fy)) continue;
     const float ws = mode == 0 ? 1.f : (mode == 1 ? __ldg(metric + (size_t)n * hw + pix) : expf(__ldg(metric + (size_t)n * hw + pix)));
-    const int x0 = (int)floorf(fx), y0 = (int)floorf(fy);
+    int x0, y0;
+    if (!splat_corner(fx, fy, W, H, x0, y0)) continue;
     const int x1 = x0 + 1, y1 = y0 + 1;
     const float wnw = ((float)x1 - fx) * ((float)y1 - fy);
     const float wne = (fx - (float)x0) * ((float)y1 - fy);
@@ -284,7 +298,8 @@ __global__ void softsplat_nhwc_kernel(const float* __restrict__ in, const float*
     const float fy = (float)y + __ldg(flow + ((size_t)n * 2 + 1) * hw + pix);
     if (!isfinite(fx) || !isfinite(fy)) continue;  // softsplat.py:158-159
     const float ws = mode == 0 ? 1.f : (mode == 1 ? __ldg(metric + pid) : expf(__ldg(metric + pid)));
-    const int x0 = (int)floorf(fx), y0 = (int)floorf(fy);
+    int x0, y0;
+    if (!splat_corner(fx, fy, W, H, x0, y0)) continue;
     const int x1 = x0 + 1, y1 = y0 + 1;
     const float wnw = ((float)x1 - fx) * ((float)y1 - fy);
     const float wne = (fx - (float)x0) * ((float)y1 - fy);
@@ -489,12 +504,9 @@ cudaError_t launch_softsplat_weighted(const float* in, const float* flow, const 
   return cudaGetLastError();
 }
 
-cudaError_t launch_volume81(bool dot, const float* one, const float* two, float* out, int N, int C, int H, int W,
-                            cudaStream_t st) {
-  static const bool tiled = [] {  // VFI_OPS_TILED=0: the first-version per-pixel kernels (A/B runs)
-    const char* e = std::getenv("VFI_OPS_TILED");
-    return !(e && e[0] == '0');
-  }();
+// tiled = false: the first-version per-pixel kernels; N > 65535 (more images than grid.z holds) takes them as well
+cudaError_t launch_volume81_form(bool tiled, bool dot, const float* one, const float* two, float* out, int N, int C, int H, int W,
+                                 cudaStream_t st) {
   if (tiled && N <= 65535) {
     const dim3 g((unsigned)((W + 31) / 32), (unsigned)((H + 7) / 8), (unsigned)N);
     if (dot)
@@ -509,6 +521,15 @@ cudaError_t launch_volume81(bool dot, const float* one, const float* two, float*
   else
     VFI_LAUNCH((volume81_kernel<false>), grid_for(total, 128), 128, 0, st, one, two, out, N, C, H, W);
   return cudaGetLastError();
+}
+
+cudaError_t launch_volume81(bool dot, const float* one, const float* two, float* out, int N, int C, int H, int W,
+                            cudaStream_t st) {
+  static const bool tiled = [] {  // VFI_OPS_TILED=0: the first-version per-pixel kernels (A/B runs)
+    const char* e = std::getenv("VFI_OPS_TILED");
+    return !(e && e[0] == '0');
+  }();
+  return launch_volume81_form(tiled, dot, one, two, out, N, C, H, W, st);
 }
 
 // channel-last forms: `sa` / `sb` are caller-provided scratch of N * H * W * round4(C) floats each (context-owned)
@@ -546,13 +567,10 @@ cudaError_t launch_volume81_warp(bool dot, const float* one, const float* two, f
   return cudaGetLastError();
 }
 
-cudaError_t launch_sepconv(const float* in, const float* ver, const float* hor, float* out, int N, int C, int H, int W,
-                           int Kv, int Kh, cudaStream_t st) {
+// py = 0: the first-version per-pixel kernel, 1 - 3: the tiled K = 51 kernel with py pixels per thread
+cudaError_t launch_sepconv_form(int py, const float* in, const float* ver, const float* hor, float* out, int N, int C, int H, int W,
+                                int Kv, int Kh, cudaStream_t st) {
   // the reference's only kernel size is 51 (sepconv_enhanced.py: 51-tap heads): shared-memory tiled fast path
-  static const int py = [] {  // VFI_SEPCONV_PY = 0 (first-version kernel), 1, 2 (default) or 3 pixels per thread
-    const char* e = std::getenv("VFI_SEPCONV_PY");
-    return (e && e[0] >= '0' && e[0] <= '3') ? e[0] - '0' : 2;
-  }();
   if (Kv == 51 && Kh == 51 && py > 0 && N <= 65535) {
     auto go = [&](auto kern, int PY) -> cudaError_t {
       const size_t smem = (size_t)(8 * PY + 50) * (32 + 50) * sizeof(float4);
@@ -573,6 +591,15 @@ cudaError_t launch_sepconv(const float* in, const float* ver, const float* hor, 
     if (e != cudaSuccess) return e;
   }
   return cudaSuccess;
+}
+
+cudaError_t launch_sepconv(const float* in, const float* ver, const float* hor, float* out, int N, int C, int H, int W,
+                           int Kv, int Kh, cudaStream_t st) {
+  static const int py = [] {  // VFI_SEPCONV_PY = 0 (first-version kernel), 1, 2 (default) or 3 pixels per thread
+    const char* e = std::getenv("VFI_SEPCONV_PY");
+    return (e && e[0] >= '0' && e[0] <= '3') ? e[0] - '0' : 2;
+  }();
+  return launch_sepconv_form(py, in, ver, hor, out, N, C, H, W, Kv, Kh, st);
 }
 
 }  // namespace vfi

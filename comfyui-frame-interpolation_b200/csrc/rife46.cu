@@ -176,6 +176,7 @@ struct vfi_ctx {
   DevBuf dbgF, dbgM;
   cudaStream_t s_h2d = nullptr, s_comp = nullptr, s_d2h = nullptr;
   DevBuf ops_a, ops_b;           // scratch of the channel-last op kernels (splat, 9 x 9 volumes)
+  cudaEvent_t ops_done = nullptr;  // recorded on the stream of the last call that used ops_a / ops_b (ops_scratch_acquire)
   vfi::PinnedBuf pin_in, pin_out;
   // per-kernel-group timing of the forward schedule (vfi_rife_profile): CUDA events recorded on the launching stream
   // around each group while `profile` is set; read (and summed per group id) by vfi_rife_profile_read
@@ -704,6 +705,7 @@ int vfi_create(int device, vfi_ctx** out) {
   CK(cudaStreamCreateWithFlags(&c->s_h2d, cudaStreamNonBlocking));
   CK(cudaStreamCreateWithFlags(&c->s_comp, cudaStreamNonBlocking));
   CK(cudaStreamCreateWithFlags(&c->s_d2h, cudaStreamNonBlocking));
+  CK(cudaEventCreateWithFlags(&c->ops_done, cudaEventDisableTiming));
   *out = c;
   return VFI_OK;
 }
@@ -730,6 +732,7 @@ int vfi_destroy(vfi_ctx* c) {
   if (c->s_h2d) cudaStreamDestroy(c->s_h2d);
   if (c->s_comp) cudaStreamDestroy(c->s_comp);
   if (c->s_d2h) cudaStreamDestroy(c->s_d2h);
+  if (c->ops_done) cudaEventDestroy(c->ops_done);
   delete c;
   return VFI_OK;
 }
@@ -1311,6 +1314,22 @@ int vfi_warp_bilinear_border(vfi_ctx* c, const float* img, const float* flow, fl
   return VFI_OK;
 }
 
+// ops_a / ops_b belong to the context, not to a stream, and the op entry points run on whatever stream the caller passes.
+// A call that uses them first makes its stream wait for the previous user (ops_done), and after its launches records
+// ops_done on its own stream, so calls on different streams take turns on the scratch instead of overwriting each other's.
+// Growing the buffers frees the old ones, so a regrowth first waits on the host for the previous user to finish.
+static cudaError_t ops_scratch_acquire(vfi_ctx* c, size_t bytes, cudaStream_t st) {
+  cudaError_t e;
+  if (bytes > c->ops_a.cap || bytes > c->ops_b.cap) {
+    if ((e = cudaEventSynchronize(c->ops_done)) != cudaSuccess) return e;
+    if ((e = c->ops_a.ensure(bytes)) != cudaSuccess) return e;
+    if ((e = c->ops_b.ensure(bytes)) != cudaSuccess) return e;
+  }
+  return cudaStreamWaitEvent(st, c->ops_done, 0);
+}
+
+static cudaError_t ops_scratch_release(vfi_ctx* c, cudaStream_t st) { return cudaEventRecord(c->ops_done, st); }
+
 int vfi_softsplat_sum(vfi_ctx* c, const float* in, const float* flow, float* out, int N, int C, int H, int W,
                       void* stream) {
   if (!c || !in || !flow || !out || N < 1 || C < 1 || H < 1 || W < 1) return fail(VFI_E_INVALID, "bad argument");
@@ -1330,11 +1349,10 @@ int vfi_softsplat_weighted(vfi_ctx* c, const float* in, const float* flow, const
     return !(e && e[0] == '0');
   }();
   if (nhwc && N <= 65535) {
-    const size_t fl = ops_scratch_floats(N, C, H, W) * sizeof(float);
-    CK(c->ops_a.ensure(fl));
-    CK(c->ops_b.ensure(fl));
-    CK(launch_softsplat_weighted_nhwc(in, flow, metric, mode, eps, out, norm, (float*)c->ops_a.p, (float*)c->ops_b.p, N, C, H, W,
-                                      static_cast<cudaStream_t>(stream)));
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    CK(ops_scratch_acquire(c, ops_scratch_floats(N, C, H, W) * sizeof(float), st));
+    CK(launch_softsplat_weighted_nhwc(in, flow, metric, mode, eps, out, norm, (float*)c->ops_a.p, (float*)c->ops_b.p, N, C, H, W, st));
+    CK(ops_scratch_release(c, st));
     c->launches += 3;
     return VFI_OK;
   }
@@ -1356,10 +1374,10 @@ int vfi_costvol_l1(vfi_ctx* c, const float* one, const float* two, float* out, i
     return e && e[0] == '1';
   }();
   if (warp_form && N <= 65535 && H <= 65535) {
-    const size_t fl = ops_scratch_floats(N, C, H, W) * sizeof(float);
-    CK(c->ops_a.ensure(fl));
-    CK(c->ops_b.ensure(fl));
-    CK(launch_volume81_warp(false, one, two, out, (float*)c->ops_a.p, (float*)c->ops_b.p, N, C, H, W, (cudaStream_t)stream));
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    CK(ops_scratch_acquire(c, ops_scratch_floats(N, C, H, W) * sizeof(float), st));
+    CK(launch_volume81_warp(false, one, two, out, (float*)c->ops_a.p, (float*)c->ops_b.p, N, C, H, W, st));
+    CK(ops_scratch_release(c, st));
     c->launches += 3;
     return VFI_OK;
   }
@@ -1380,10 +1398,10 @@ int vfi_corr_dot(vfi_ctx* c, const float* first, const float* second, float* out
     return e && e[0] == '1';
   }();
   if (warp_form && N <= 65535 && H <= 65535) {
-    const size_t fl = ops_scratch_floats(N, C, H, W) * sizeof(float);
-    CK(c->ops_a.ensure(fl));
-    CK(c->ops_b.ensure(fl));
-    CK(launch_volume81_warp(true, first, second, out, (float*)c->ops_a.p, (float*)c->ops_b.p, N, C, H, W, (cudaStream_t)stream));
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    CK(ops_scratch_acquire(c, ops_scratch_floats(N, C, H, W) * sizeof(float), st));
+    CK(launch_volume81_warp(true, first, second, out, (float*)c->ops_a.p, (float*)c->ops_b.p, N, C, H, W, st));
+    CK(ops_scratch_release(c, st));
     c->launches += 3;
     return VFI_OK;
   }

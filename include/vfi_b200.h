@@ -113,7 +113,9 @@ int vfi_softsplat_sum(vfi_ctx* ctx, const float* in, const float* flow, float* o
                       void* stream);
 /* Fused form of the wrapper modes of softsplat() (cupy_ops/softsplat.py:382-435): mode 0 avg, 1 linear, 2 soft (weight 1,
  * metric, exp(metric) per source pixel), eps 0 addeps (default) / 1 zeroeps / 2 clipeps; `norm` is a caller-provided
- * [N,1,H,W] scratch plane (the splatted weights); out [N,C,H,W] = splat(in * weight) / f(norm).  metric may be NULL for avg. */
+ * [N,1,H,W] scratch plane (the splatted weights); out [N,C,H,W] = splat(in * weight) / f(norm).  metric may be NULL for avg.
+ * The splat and the channel-last volume form use scratch owned by the context; calls on different streams are ordered
+ * against each other on it (the later call's stream waits for the earlier call), so one context may serve several streams. */
 int vfi_softsplat_weighted(vfi_ctx* ctx, const float* in, const float* flow, const float* metric, int mode, int eps, float* out,
                            float* norm, int N, int C, int H, int W, void* stream);
 int vfi_costvol_l1(vfi_ctx* ctx, const float* one, const float* two, float* out, int N, int C, int H, int W,

@@ -31,4 +31,12 @@ int emu_volume81(int dot, const float* one, const float* two, float* out, int N,
 int emu_sepconv(const float* in, const float* ver, const float* hor, float* out, int N, int C, int H, int W, int Kv, int Kh) {
   return (int)vfi::launch_sepconv(in, ver, hor, out, N, C, H, W, Kv, Kh, nullptr);
 }
+// the forms that VFI_OPS_TILED / VFI_SEPCONV_PY select, chosen per call (the environment is read once per process)
+int emu_volume81_form(int tiled, int dot, const float* one, const float* two, float* out, int N, int C, int H, int W) {
+  return (int)vfi::launch_volume81_form(tiled != 0, dot != 0, one, two, out, N, C, H, W, nullptr);
+}
+int emu_sepconv_form(int py, const float* in, const float* ver, const float* hor, float* out, int N, int C, int H, int W, int Kv,
+                     int Kh) {
+  return (int)vfi::launch_sepconv_form(py, in, ver, hor, out, N, C, H, W, Kv, Kh, nullptr);
+}
 }

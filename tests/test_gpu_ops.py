@@ -5,6 +5,7 @@ import pytest
 import torch
 
 from oracle import ops_ref as R
+from ops_cases import first_mismatch
 
 pytestmark = pytest.mark.gpu
 
@@ -31,7 +32,10 @@ def test_softsplat_modes(ops):
         for mode in ("sum", "avg", "linear", "soft", "soft-zeroeps", "linear-clipeps"):
             m = None if mode in ("sum", "avg") else (metric.abs() + 0.1 if "linear" in mode else metric)
             got = ops.softsplat(x.cuda(), flow.cuda(), None if m is None else m.cuda(), mode)
-            assert _close(got, R.softsplat(x, flow, m, mode), 1e-4), mode
+            ref = R.softsplat(x, flow, m, mode)
+            # summation order and exp differ from the oracle, nothing else: measured <= 4.8e-7 on the host build
+            err = first_mismatch(got, ref, (2e-5 if mode == "sum" else 2e-6) * max(1.0, float(ref.abs().max())))
+            assert err is None, f"{(c, h, w)} {mode}: {err}"
 
 
 def test_costvol_and_correlation(ops):

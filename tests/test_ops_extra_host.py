@@ -10,6 +10,7 @@ import pytest
 import torch
 
 from oracle import ops_ref
+from ops_cases import ADACOF_SHAPES, adacof_inputs, first_mismatch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CUDA_INC = "/usr/local/cuda/include"
@@ -54,3 +55,14 @@ def test_edt_pass_kernel(emu):
     out = torch.zeros_like(data)
     assert emu.emu_edt_pass(vp(data), vp(out), 3, 10, 17, C.c_float(diam2)) == 0
     assert torch.equal(out, ops_ref.edt_pass(data, diam2))
+
+
+@pytest.mark.parametrize("shape", ADACOF_SHAPES, ids=lambda s: "x".join(map(str, s)))
+def test_adacof_exact(emu, shape):
+    """dyadic inputs (tests/ops_cases.py), offsets in [-6, 6] with negative fractions: bit-exact against the oracle"""
+    n, c, ho, wo, f, dil = shape
+    x, w, oi, oj = adacof_inputs(n, c, ho, wo, f, dil, sum(shape))
+    out = torch.full((n, c, ho, wo), float("nan"))
+    assert emu.emu_adacof(vp(x), vp(w), vp(oi), vp(oj), vp(out), n, c, x.shape[2], x.shape[3], f, dil, ho, wo) == 0
+    err = first_mismatch(out, ops_ref.adacof(x, w, oi, oj, dil))
+    assert err is None, err
